@@ -2,7 +2,8 @@
 """bench.py -- headline benchmark of the B200 wavelet filterbank engine.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference|aten] [--config headline|c5]
-    (N>1: launched by the driver as  python -m torch.distributed.run --nproc-per-node N bench.py --gpus N ...)
+                    [--dump-outputs DIR]
+    (N>1: run as  python -m torch.distributed.run --nproc-per-node N bench.py --gpus N ...)
 
 One "step" = one pass of the hot path over one batch of synthetic input:
     DWTForward(J=3,'db4','symmetric') on randn(128,32,512,512)          (BASELINE.json configs[1])
@@ -28,6 +29,9 @@ Also on the JSON line:
                    gather + depthwise F.conv2d + slicing), i.e. the "existing kernels" bar on the same B200.
 --config c5      : BASELINE.json configs[4]: DWTForward J=4 db8 (zero) on N=1024, C=16, 2048x2048, sharded over N,
                    streamed through the GPUs in chunks; yl is all-gathered at the end (the band-passes stay rank-resident).
+--dump-outputs DIR : after the timed steps, write what the last step returned (yl and every yh[j] of both transforms,
+                   rank 0) as DIR/<name>.npy, float32; see dump_outputs().  The inputs are seeded, so two builds run with
+                   the same arguments can be compared output for output.  Headline config of --impl ours only.
 """
 import argparse
 import json
@@ -62,7 +66,13 @@ def parse():
     ap.add_argument('--dtcwt-batch', type=int, default=DTCWT_SHAPE[0])
     ap.add_argument('--c5-n-total', type=int, default=1024)
     ap.add_argument('--c5-chunk', type=int, default=16)
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None)
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error('--steps must be at least 1')
+    if a.dump_outputs is not None and (a.impl != 'ours' or a.config != 'headline'):
+        ap.error('--dump-outputs is only supported for the headline config of --impl ours')
+    return a
 
 
 def load_peaks():
@@ -299,6 +309,26 @@ def timed(torch, fn, reps, warm=2):
     return e0.elapsed_time(e1) / reps
 
 
+DUMP_CAP = 1 << 20   # elements per dumped array: the 8 arrays of a step stay under 64 MB
+
+
+def dump_outputs(torch, out_dir, arrays):
+    """Write each (name, tensor) as out_dir/<name>.npy in float32.  A tensor of at most DUMP_CAP elements is written
+    whole, with its shape; a larger one as the 1-D array of DUMP_CAP of its elements, taken in flat (C) order at
+    positions drawn without replacement by a generator seeded from the name, so that every run and every build with
+    the same shapes samples the same elements."""
+    import zlib
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays:
+        t = t.detach()
+        if t.numel() > DUMP_CAP:
+            rng = np.random.default_rng(zlib.crc32(name.encode()))
+            idx = np.sort(rng.choice(t.numel(), DUMP_CAP, replace=False))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        np.save(os.path.join(out_dir, name + '.npy'), t.cpu().numpy().astype(np.float32))
+
+
 def run_ours(args):
     torch, dist, world, rank, local, dev, numa = setup_dist(args)
     import pytorch_wavelets_b200 as pw
@@ -348,6 +378,10 @@ def run_ours(args):
     calls = rec.summary()
     launches = rec.count
     kernels_per_step = 3 + 3   # DWT: pyramid level 1 + 2 streaming levels; DTCWT: 3 levels (see DESIGN.md section 4)
+    if args.dump_outputs is not None and rank == 0:
+        dump_outputs(torch, args.dump_outputs,
+                     [('dwt_yl', a[0])] + [('dwt_yh%d' % j, h) for j, h in enumerate(a[1])] +
+                     [('dtcwt_yl', b[0])] + [('dtcwt_yh%d' % j, h) for j, h in enumerate(b[1])])
     del a, b
 
     tt = torch.tensor([t_d + t_t, t_d, t_t], device=dev, dtype=torch.float64)
